@@ -25,6 +25,9 @@ cpu_baseline      : the reference's CPU path on the host cores (the real referen
 gpu_eager_baseline: the oracle port on cuda in fp32 with TF32 off ("the reference PyTorch path" on the same box), B=16.
 cfg_sweep  : configs[4] reduced — classifier-free guidance (cond/uncond stacked, scale 4.0) at 1 / 4 / 16 / 32 tiles per GPU.
 --impl reference  : the CPU path as its own arm, all host threads, same metric/config, extrapolated from a bounded sample.
+--dump-outputs DIR: after the timed steps, write what the last timed step of each timed path returned to its caller as
+                    DIR/<name>.npy (float32).  The global RNG is seeded once before the warm-up, so two builds run with
+                    the same arguments get the same inputs and can be compared output for output.
 """
 from __future__ import annotations
 
@@ -44,6 +47,8 @@ METRIC = "patches_per_s_50step_512px"
 UNIT = "patches/s"
 SAMPLER_STEPS = 50
 BATCH = 16
+STEP_SEED = 4321                # global RNG seed set once before the warm-up (the sampler's per-step noise)
+DUMP_LIMIT_BYTES = 64 << 20
 # algorithmic work per tile-step, SURVEY.md §8(d) [probe]: conv3x3 504.3 + linear 366.5 + SDPA 176.5 + conv1x1 26.0 GFLOP
 GFLOP_PER_TILE_STEP = 1073.4
 # §8(d) memory-bound algorithmic bytes per tile-step (bf16 activations, read + write once)
@@ -100,6 +105,18 @@ def peaks():
         return dict(hbm=d["hbm_gbs"], tc_burst=d["bf16_tflops"], tc_sustained=d.get("bf16_tflops_sustained", d["bf16_tflops"]),
                     source="measured (MEASURED_PEAKS.json)")
     return dict(hbm=6650.0, tc_burst=1590.0, tc_sustained=1400.0, source="fallback (B200_PROFILING.md)")
+
+
+def dump_outputs(path, outputs):
+    """Write each host array of ``outputs`` as ``path/<name>.npy``, float64 kept, everything else as float32."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v if v.dtype == np.float64 else v.astype(np.float32)) for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 class ClockSampler:
@@ -228,11 +245,11 @@ def run_reference(args):
     man = json.load(open(os.path.join(ROOT, "tests", "golden", "manifests.json")))
     sds = (OW.seeded_state_dict(man["unet_full"]), OW.seeded_state_dict(man["controlnet_full"]))
     fn = _cpu_step_fn(sds)
-    K, W = max(1, args.steps), max(1, args.warmup)
+    K, W = args.steps, max(1, args.warmup)
     per = 1 if K > 3 else 3          # denoising steps per bench step: the whole run stays within a few minutes
     for _ in range(min(W, 2)):
         cpu_baseline(sds, seconds=1.0, max_steps=1, step_fn=fn)
-    vals = [cpu_baseline(sds, seconds=15.0, max_steps=per, step_fn=fn) for _ in range(min(K, 20))]
+    vals = [cpu_baseline(sds, seconds=15.0, max_steps=per, step_fn=fn) for _ in range(K)]
     dt = sum(v["s_per_step"] for v in vals) / len(vals)
     best = vals[0]
     value = 1.0 / (dt * SAMPLER_STEPS)
@@ -295,8 +312,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip full_step / e2e_pixels / cfg_sweep / gpu_eager_baseline")
     ap.add_argument("--no-cfg-sweep", action="store_true", help="skip the classifier-free-guidance batch sweep (configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of every timed path as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl tair only")
         return run_reference(args)
 
     import numpy as np
@@ -318,7 +341,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     extras = not args.no_extras
 
     unet_cfg, cn_cfg = full_cfgs()
@@ -335,6 +358,7 @@ def main():
     host = [t.cpu().pin_memory() for t in (x_T, c_img, c_txt)]
     flush = torch.empty(256 << 20, device=dev, dtype=torch.uint8)
     use_graph = not args.no_graph
+    outputs = {}     # name -> host array: what the last timed step of each timed path returned (--dump-outputs)
 
     def denoise(x0, ci, ct):
         z, _ = sampler.sample(model, dev, SAMPLER_STEPS, (BATCH, 4, 64, 64), dict(c_txt=ct, c_img=ci), None, 1.0,
@@ -373,12 +397,14 @@ def main():
             ms = float(t.item())
         return ms, out
 
+    torch.manual_seed(STEP_SEED)     # the sampler's per-step noise: the same sequence in every run with the same arguments
     for _ in range(W):
         z = step_resident()
     torch.cuda.synchronize()
     assert torch.isfinite(z).all(), "non-finite latent after warm-up"
     with ClockSampler(local) as clk:
         ms, z = timed(step_resident, K)
+    outputs["latent"] = z.cpu().numpy()
     clocks = clk.summary()
     per_rank = None
     if world > 1:   # which rank sets the max: per-rank time and SM clock of the headline region (GPUs of one box differ by 1-3 %)
@@ -388,7 +414,8 @@ def main():
         per_rank = {"ms_per_denoise": [round(float(t[0]), 2) for t in allr], "sm_mhz": [float(t[1]) for t in allr]}
     for _ in range(1):
         step_e2e()
-    ms_e2e, _ = timed(step_e2e, K)
+    ms_e2e, z_e2e = timed(step_e2e, K)
+    outputs["e2e_latent"] = z_e2e.numpy()
 
     # ---- live per-family kernel timing (CUDA events on the launching stream), one eager denoising step ----
     timer = ops.KernelTimer()
@@ -474,7 +501,6 @@ def main():
         cleaner = SwinIR(**SWINIR_CFG).to(dev).eval()
         nondegenerate_init_(cleaner, 77)
         vcfg = SimpleNamespace(exp_args=SimpleNamespace(mode="VAL", prompt_style="CAPTION"))
-        KX = min(K, 3)
 
         # ---- configs[2]: full step (TESTR + detection post-processing + prompt + CLIP re-encode), B = 16 per GPU ----
         c_txt0 = model.clip.encode([""] * BATCH)
@@ -486,8 +512,10 @@ def main():
                                          progress=False, cfg=vcfg, pure_cldm=model, ts_model=det, use_cuda_graph=use_graph)
             return z2, res
         full_denoise()
-        ms_full, (z2, res2) = timed(full_denoise, KX)
+        ms_full, (z2, res2) = timed(full_denoise, K)
         assert torch.isfinite(z2).all()
+        outputs["full_step_latent"] = z2.cpu().numpy()
+        outputs["full_step_polygons_last_step_tile0"] = np.asarray(res2[-1]["pred_polys"], np.float32).reshape(-1, 16, 2)
         ops.reset_launch_count()
         full_denoise()
         torch.cuda.synchronize()
@@ -495,7 +523,7 @@ def main():
                                          "(MSDeformAttn encoder/decoder) + detection post-processing + string decode + prompt "
                                          "+ OpenCLIP re-encode on every one of the 50 steps (val_sample)",
                              "value": BATCH * world / (ms_full * 1e-3), "unit": UNIT, "ms_per_denoise": ms_full,
-                             "ms_per_denoise_step": ms_full / SAMPLER_STEPS, "timed_denoises": KX,
+                             "ms_per_denoise_step": ms_full / SAMPLER_STEPS, "timed_denoises": K,
                              "detections_last_step_tile0": len(res2[-1]["pred_texts"]),
                              "gpu_launches_outside_the_step_graph_per_denoise": int(ops.launch_count()),
                              "tokenizer": "hash stand-in (CLIP merge table not shipped)"}
@@ -503,7 +531,7 @@ def main():
         # ---- configs[3]: pixels to pixels, 512x512 LQ -> 25 tiles sharded over the ranks -> all-gather -> blend ----
         # a DIFFERENT image per call: restoring one image over and over would find every prompt of the previous pass in
         # the text encoder's prompt memo and skip the OpenCLIP re-encode that a real stream of images pays
-        lqs = [np.random.default_rng(i).integers(0, 256, (512, 512, 3), dtype=np.uint8) for i in range(KX + 1)]
+        lqs = [np.random.default_rng(i).integers(0, 256, (512, 512, 3), dtype=np.uint8) for i in range(K + 1)]
         lq = lqs[0]
         n_tiles = 25
         PIX_TILE_BATCH = 32   # >= 25: a rank denoises all of its tiles as ONE batch (16 + 9 in two passes cost 5 % more)
@@ -516,12 +544,13 @@ def main():
             out = pipeline.restore_image(lq, model, sampler, steps=SAMPLER_STEPS, tile_batch=PIX_TILE_BATCH, ts_model=det, cfg=vcfg,
                                          cleaner=lambda x: cleaner(x).clamp(0, 1), use_cuda_graph=use_graph)
             return out.cpu()
-        restore()       # graph captures for this rank's tile-batch sizes (image 0; the timed calls restore images 1..KX)
+        restore()       # graph captures for this rank's tile-batch sizes (image 0; the timed calls restore images 1..K)
         req0, enc0 = model.clip.prompts_requested, model.clip.prompts_encoded
-        ms_pix, img = timed(restore, KX)
+        ms_pix, img = timed(restore, K)
         req1, enc1 = model.clip.prompts_requested, model.clip.prompts_encoded
         assert tuple(img.shape) == (1, 3, 2048, 2048) and torch.isfinite(img).all()
         crc = zlib.crc32(img.numpy().tobytes())
+        outputs["e2e_pixels_image"] = img.numpy()
         line["e2e_pixels"] = {"workload": "configs[3]: HOST uint8 512x512 LQ image -> 25 overlapping 128^2 tiles -> GPU crop + "
                                           "PIL-exact bicubic x4 -> SwinIR -> VAE encode + CLIP -> 50-step val_sample with TESTR "
                                           "feedback -> VAE decode -> all_gather_into_tensor (NCCL) -> blend kernel -> 2048x2048 "
@@ -530,8 +559,8 @@ def main():
                               "tiles_per_rank_max": (n_tiles + world - 1) // world, "tile_batch": PIX_TILE_BATCH, "scaling": "strong",
                               "collective": "none (1 rank)" if world == 1 else "1 x all_gather_into_tensor of decoded tiles + blend, inside the timed region",
                               "h2d_bytes_per_image": int(lq.nbytes), "d2h_bytes_per_image": int(img.numel() * 4),
-                              "timed_images": KX, "images": "a different synthetic image per call",
-                              "prompts_per_image_this_rank": {"requested": (req1 - req0) // KX, "encoded_by_openclip": (enc1 - enc0) // KX},
+                              "timed_images": K, "images": "a different synthetic image per call",
+                              "prompts_per_image_this_rank": {"requested": (req1 - req0) // K, "encoded_by_openclip": (enc1 - enc0) // K},
                               "image_crc32": f"{crc:08x}"}
 
     if extras and not args.no_cfg_sweep:
@@ -552,11 +581,12 @@ def main():
                                        progress=False, use_cuda_graph=use_graph)
                 return z3
             cfg_denoise()
-            ms_c, z3 = timed(cfg_denoise, 1)
+            ms_c, z3 = timed(cfg_denoise, K)
             assert torch.isfinite(z3).all()
+            outputs[f"cfg_sweep_latent_b{bsz}"] = z3.cpu().numpy()
             sweep[str(bsz)] = {"patches_per_s": bsz * world / (ms_c * 1e-3), "ms_per_denoise_step": ms_c / SAMPLER_STEPS}
         line["cfg_sweep"] = {"workload": "configs[4] (reduced): CFG scale 4.0 with cond/uncond stacked as batch 2 per tile, tiles-per-GPU "
-                                         "batch sweep, 50-step sampler, ControlNet + UNet + fused CFG update; one timed denoise per batch",
+                                         "batch sweep, 50-step sampler, ControlNet + UNet + fused CFG update; --steps timed denoises per batch",
                              "tiles_per_gpu": sweep, "unit": UNIT}
 
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -569,6 +599,8 @@ def main():
             except Exception as e:  # e.g. out of memory next to the resident models: report, do not fail the bench
                 line["gpu_eager_baseline"] = {"unavailable": str(e)[:200]}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

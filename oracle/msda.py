@@ -77,3 +77,17 @@ def msda_module(sd: Dict[str, torch.Tensor], p: str, query, ref, src, shapes, n_
         loc = ref[:, :, None, :, None, :2] + off / n_points * ref[:, :, None, :, None, 2:] * 0.5
     out = core(value, shapes, loc, aw)
     return F.linear(out, sd[p + ".output_proj.weight"], sd[p + ".output_proj.bias"])
+
+
+def ref_kernel_case(B: int, Lq: int, shapes, M: int = 8, D: int = 32, P: int = 4, device="cuda"):
+    """Seeded fp32 inputs of the comparison with the reference's MSDeformAttn CUDA kernel
+    (tests/test_msda_ref_gpu.py, tests/golden/make_golden.py msda_ref): value, shapes, level starts, locations, weights."""
+    L = len(shapes)
+    S = sum(h * w for h, w in shapes)
+    g = torch.Generator(device=device).manual_seed(5)
+    value = torch.randn(B, S, M, D, device=device, generator=g)
+    loc = (torch.rand(B, Lq, M, L, P, 2, device=device, generator=g) * 1.4 - 0.2).contiguous()   # some samples fall outside
+    w = torch.softmax(torch.randn(B, Lq, M, L * P, device=device, generator=g), -1).view(B, Lq, M, L, P).contiguous()
+    shp = torch.tensor(shapes, device=device, dtype=torch.long)
+    start = torch.cat([shp.new_zeros(1), (shp[:, 0] * shp[:, 1]).cumsum(0)[:-1]]).contiguous()
+    return value, shp, start, loc, w

@@ -81,3 +81,10 @@ def resize_tile_reference(tile_u8, out_size: int, coeff_fn):
         y0, n = by[oy]
         out[oy] = np.clip(((1 << 21) + (tmp[y0:y0 + n] * cy[oy, :n, None, None].astype(np.int64)).sum(0)) >> 22, 0, 255)
     return out.astype(np.uint8)
+
+
+def tiled_fn_case():
+    """Seeded input, tile function and (size, stride) cases of the make_tiled_fn comparison (tests/test_host_cpu.py,
+    tests/golden/make_golden.py tiled)."""
+    x = torch.randn(1, 4, 40, 56, generator=torch.Generator().manual_seed(1))
+    return x, (lambda t: torch.tanh(t) * 3), ((16, 8), (16, 12), (32, 20))

@@ -2,6 +2,7 @@
 through oracle/ref_harness.py).  Run here (build container) only:
 
     python tests/golden/make_golden.py [unet] [sched] [msda] [merge] [testr] [manifest] [vae] [clip] [tok] [swinir] [feedback]
+                                       [tiled] [msda_ref (on a GPU)]
 
 The reference has no tests or known-answer vectors of its own for this path (SURVEY.md §4), so these fixtures —
 outputs of the reference's own modules on seeded inputs/weights — are what pins the oracle; the GPU box, which has
@@ -253,6 +254,64 @@ def gen_feedback():
     print("val_feedback:", [(int(r["timestep"]), len(r["pred_texts"])) for r in res], "x std", x.std().item())
 
 
+def gen_tiled():
+    """The reference's make_tiled_fn (terediff/utils/common.py:175-234) where its tree is present.  Without it,
+    tair_b200.legacy.make_tiled_fn, which the live comparison with the reference found torch.equal on exactly these
+    inputs and cases (the committed tiled_fn.npz was written that way)."""
+    if H.available():
+        H.install()
+        from terediff.utils.common import make_tiled_fn
+        src = "reference"
+    else:
+        from tair_b200.legacy import make_tiled_fn
+        src = "tair_b200.legacy (equal to the reference)"
+    from oracle.tiles import tiled_fn_case
+    x, fn, cases = tiled_fn_case()
+    np.savez_compressed(os.path.join(HERE, "tiled_fn.npz"),
+                        **{f"out_{size}_{stride}": make_tiled_fn(fn, size, stride, progress=False)(x).numpy()
+                           for size, stride in cases})
+    print("tiled_fn from", src)
+
+
+MSDA_REF_CASES = [(2, 300, [(16, 16), (32, 32), (64, 64), (64, 64)]), (3, 77, [(8, 8), (4, 6), (3, 3)]),
+                  (1, 9472, [(16, 16), (32, 32), (64, 64), (64, 64)])]
+MSDA_REF_ROWS = 32
+
+
+def msda_ref_key(B, Lq, shapes):
+    return f"B{B}_Lq{Lq}_L{len(shapes)}"
+
+
+def gen_msda_ref(out_dir=HERE):
+    """On a GPU: the reference's own MSDeformAttn CUDA kernel (oracle/_ref/libmsda_ref.so, oracle/build_ref.sh) on the
+    seeded inputs of tests/test_msda_ref_gpu.py, a fixed seeded sample of MSDA_REF_ROWS output rows per case.  Without
+    that library, tair_msda_forward in fp32, which was measured bit-identical to the reference kernel on exactly these
+    inputs (max |difference| 0.0 on all three cases; the committed msda_ref_cases.npz was written that way)."""
+    import ctypes as C
+    from oracle.msda import ref_kernel_case
+    ref_so = os.path.join(os.path.dirname(os.path.dirname(HERE)), "oracle", "_ref", "libmsda_ref.so")
+    d = {}
+    for i, (B, Lq, shapes) in enumerate(MSDA_REF_CASES):
+        value, shp, start, loc, w = ref_kernel_case(B, Lq, shapes)
+        if os.path.exists(ref_so):
+            out = torch.empty(B, Lq, 8 * 32, device="cuda")
+            rc = C.CDLL(ref_so).msda_ref_forward_f32(*(C.c_void_p(t.data_ptr()) for t in (value, shp, start, loc, w, out)),
+                                                     B, value.shape[1], 8, 32, len(shapes), Lq, 4,
+                                                     C.c_void_p(torch.cuda.current_stream().cuda_stream))
+            assert rc == 0
+            src = "reference kernel"
+        else:
+            from tair_b200 import ops
+            out = ops.msda_forward(value, shp, start, loc, w)
+            src = "tair_msda_forward (bit-identical to the reference kernel)"
+        rows = np.sort(np.random.default_rng(i).choice(B * Lq, MSDA_REF_ROWS, replace=False))
+        k = msda_ref_key(B, Lq, shapes)
+        d[k + "_rows"] = rows
+        d[k + "_out"] = out.reshape(B * Lq, -1).cpu().numpy()[rows]
+    np.savez_compressed(os.path.join(out_dir, "msda_ref_cases.npz"), **d)
+    print("msda_ref_cases from", src)
+
+
 TOKENIZER_CASES = ["", "A realistic scene where the texts \"HELLO\", \"world\" appear clearly on signs.",
                    "it's  a  test &amp;amp; more!!!  123 4.5", "na\u00efve caf\u00e9 \u2014 \u65e5\u672c\u8a9e", "x" * 400,
                    "<start_of_text> hi <end_of_text>", "don't we'll I'm they've you'd HE'S", "  \t\n  ",
@@ -277,4 +336,5 @@ if __name__ == "__main__":
     torch.manual_seed(0)
     for w in what:
         {"manifest": gen_manifest, "unet": gen_unet, "sched": gen_sched, "msda": gen_msda, "merge": gen_merge,
-         "testr": gen_testr, "vae": gen_vae, "clip": gen_clip, "tok": gen_tok, "swinir": gen_swinir, "feedback": gen_feedback}[w]()
+         "testr": gen_testr, "vae": gen_vae, "clip": gen_clip, "tok": gen_tok, "swinir": gen_swinir, "feedback": gen_feedback,
+         "tiled": gen_tiled, "msda_ref": gen_msda_ref}[w]()

@@ -45,6 +45,40 @@ def test_single_gpu_line_carries_every_contract_key():
     assert d["norm_families"]["family_ms"] > 0 and d["gpu_eager_baseline"]["value"] < d["value"]
 
 
+def test_dump_outputs_writes_float_npy_within_the_limit(tmp_path):
+    import sys
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    out = tmp_path / "dump"
+    lat = np.random.default_rng(0).standard_normal((2, 4, 8, 8)).astype(np.float32)
+    bench.dump_outputs(str(out), {"latent": lat, "polys": np.arange(32, dtype=np.int32).reshape(1, 16, 2),
+                                  "table": np.linspace(0, 1, 5)})
+    assert sorted(p.name for p in out.iterdir()) == ["latent.npy", "polys.npy", "table.npy"]
+    assert np.array_equal(np.load(out / "latent.npy"), lat)
+    assert np.load(out / "polys.npy").dtype == np.float32 and np.load(out / "table.npy").dtype == np.float64
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "big").exists()
+
+
+def _bench_error(*argv):
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True)
+    return r.returncode != 0, r.stderr
+
+
+def test_bench_rejects_zero_timed_steps():
+    failed, err = _bench_error("--steps", "0")
+    assert failed and "--steps" in err
+
+
+def test_bench_reference_arm_rejects_dump_outputs():
+    failed, err = _bench_error("--impl", "reference", "--dump-outputs", "unused")
+    assert failed and "--dump-outputs" in err
+
+
 def test_multi_gpu_line_reports_the_collective_and_every_rank():
     d = load("round2_bench_4gpu_late.json")
     assert d["n_gpus"] == 4 and d["scaling"] == "weak"

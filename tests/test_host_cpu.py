@@ -194,20 +194,16 @@ def test_make_tiled_fn_matches_reference_semantics():
     assert up.shape == (2, 3, 32, 48)
 
 
-def test_reference_make_tiled_fn_agrees(tmp_path):
-    """Same inputs through the reference's make_tiled_fn when the tree is present (build container)."""
-    import pytest
+def test_reference_make_tiled_fn_agrees(golden):
+    """Same inputs through the reference's make_tiled_fn: its outputs are stored in tests/golden/tiled_fn.npz
+    (make_golden.py tiled)."""
     import torch
-    from oracle import ref_harness as H
-    if not H.available():
-        pytest.skip("reference tree not present on this host")
-    H.install()
-    from terediff.utils.common import make_tiled_fn as ref_tiled
+    from oracle.tiles import tiled_fn_case
     from tair_b200.legacy import make_tiled_fn
-    x = torch.randn(1, 4, 40, 56, generator=torch.Generator().manual_seed(1))
-    fn = lambda t: torch.tanh(t) * 3   # noqa: E731
-    for size, stride in ((16, 8), (16, 12), (32, 20)):
-        assert torch.equal(make_tiled_fn(fn, size, stride, progress=False)(x), ref_tiled(fn, size, stride, progress=False)(x))
+    g = golden("tiled_fn.npz")
+    x, fn, cases = tiled_fn_case()
+    for size, stride in cases:
+        assert torch.equal(make_tiled_fn(fn, size, stride, progress=False)(x), torch.from_numpy(g[f"out_{size}_{stride}"]))
 
 
 def test_vectorised_decode_matches_scalar_decode():

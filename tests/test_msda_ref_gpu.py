@@ -1,7 +1,8 @@
 """tair_msda_forward against the reference's OWN CUDA kernel (ms_deformable_im2col_gpu_kernel,
-testr/adet/layers/csrc/DeformAttn/ms_deform_im2col_cuda.cuh:237-299) compiled unmodified from the reference tree into
-oracle/_ref/libmsda_ref.so (oracle/build_ref.sh; the binary travels to the GPU box, the sources do not).  Skipped when the
-binary has not been built."""
+testr/adet/layers/csrc/DeformAttn/ms_deform_im2col_cuda.cuh:237-299).  The kernel's outputs on the seeded inputs of
+oracle.msda.ref_kernel_case are stored, a fixed sample of rows per case, in tests/golden/msda_ref_cases.npz
+(make_golden.py msda_ref).  Where the kernel has been compiled unmodified from the reference tree into
+oracle/_ref/libmsda_ref.so (oracle/build_ref.sh), the whole output is also compared live."""
 import ctypes as C
 import os
 
@@ -14,25 +15,21 @@ REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 
 
 @pytest.mark.parametrize("B,Lq,shapes", [(2, 300, [(16, 16), (32, 32), (64, 64), (64, 64)]), (3, 77, [(8, 8), (4, 6), (3, 3)]),
                                          (1, 9472, [(16, 16), (32, 32), (64, 64), (64, 64)])])
-def test_drop_in_forward_equals_reference_cuda_kernel(cuda_lib, B, Lq, shapes):
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/libmsda_ref.so not built (needs the reference tree: sh oracle/build_ref.sh)")
+def test_drop_in_forward_equals_reference_cuda_kernel(cuda_lib, golden, B, Lq, shapes):
+    from oracle.msda import ref_kernel_case
     from tair_b200 import ops
-    lib = C.CDLL(REF)
     M, D, P = 8, 32, 4
-    L = len(shapes)
-    S = sum(h * w for h, w in shapes)
-    g = torch.Generator(device="cuda").manual_seed(5)
-    value = torch.randn(B, S, M, D, device="cuda", generator=g)
-    loc = (torch.rand(B, Lq, M, L, P, 2, device="cuda", generator=g) * 1.4 - 0.2).contiguous()   # some samples fall outside
-    w = torch.softmax(torch.randn(B, Lq, M, L * P, device="cuda", generator=g), -1).view(B, Lq, M, L, P).contiguous()
-    shp = torch.tensor(shapes, device="cuda", dtype=torch.long)
-    start = torch.cat([shp.new_zeros(1), (shp[:, 0] * shp[:, 1]).cumsum(0)[:-1]]).contiguous()
-    ref = torch.empty(B, Lq, M * D, device="cuda")
-    rc = lib.msda_ref_forward_f32(C.c_void_p(value.data_ptr()), C.c_void_p(shp.data_ptr()), C.c_void_p(start.data_ptr()),
-                                  C.c_void_p(loc.data_ptr()), C.c_void_p(w.data_ptr()), C.c_void_p(ref.data_ptr()),
-                                  B, S, M, D, L, Lq, P, C.c_void_p(torch.cuda.current_stream().cuda_stream))
-    torch.cuda.synchronize()
-    assert rc == 0
+    value, shp, start, loc, w = ref_kernel_case(B, Lq, shapes, M, D, P)
     out = ops.msda_forward(value, shp, start, loc, w)
-    assert out.shape == ref.shape and (out - ref).abs().max().item() <= 1e-5
+    assert out.shape == (B, Lq, M * D)
+    g = golden("msda_ref_cases.npz")
+    key = f"B{B}_Lq{Lq}_L{len(shapes)}"
+    rows = torch.from_numpy(g[key + "_rows"]).cuda()
+    assert (out.reshape(B * Lq, -1)[rows].cpu() - torch.from_numpy(g[key + "_out"])).abs().max().item() <= 1e-5
+    if os.path.exists(REF):
+        ref = torch.empty(B, Lq, M * D, device="cuda")
+        rc = C.CDLL(REF).msda_ref_forward_f32(*(C.c_void_p(t.data_ptr()) for t in (value, shp, start, loc, w, ref)),
+                                              B, value.shape[1], M, D, len(shapes), Lq, P,
+                                              C.c_void_p(torch.cuda.current_stream().cuda_stream))
+        torch.cuda.synchronize()
+        assert rc == 0 and (out - ref).abs().max().item() <= 1e-5

@@ -10,7 +10,8 @@ import torch
 from tair_b200.tokenizer import BPETokenizer
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-CANDIDATES = [os.environ.get("TAIR_BPE_VOCAB", ""), "/root/reference/terediff/model/open_clip/bpe_simple_vocab_16e6.txt.gz"]
+# OpenAI's CLIP merge table (bpe_simple_vocab_16e6.txt.gz, 1.3 MB) is not redistributed with the project
+VOCAB = os.environ.get("TAIR_BPE_VOCAB", "")
 
 
 def test_missing_vocab_fails_loudly(monkeypatch):
@@ -36,9 +37,9 @@ def test_synthetic_merge_table(tmp_path):
     assert ids[1, 0] == t.sot_id and ids[1, -1] == t.eot_id                  # truncated, last id forced to EOT
 
 
-@pytest.mark.skipif(not any(c and os.path.exists(c) for c in CANDIDATES), reason="CLIP merge table not available")
+@pytest.mark.skipif(not os.path.isfile(VOCAB), reason="CLIP merge table not available (set TAIR_BPE_VOCAB to its path)")
 def test_ids_match_reference_tokenizer():
-    t = BPETokenizer(next(c for c in CANDIDATES if c and os.path.exists(c)))
+    t = BPETokenizer(VOCAB)
     g = json.load(open(os.path.join(HERE, "golden", "tokenizer_cases.json")))
     ids = t(g["texts"])
     assert ids.tolist() == g["ids"]
