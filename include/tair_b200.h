@@ -77,7 +77,9 @@ typedef struct tair_epilogue {
   int32_t rowgroup_bf16;   /* 0: fp32 rows.  1: bf16 rows, prefetched like the residual (half the L2 traffic of the fp32
                               form; TESTR's per-query positional projections).  Needs a 16-byte aligned bf16 output,
                               N % 32 == 0, rows 16-byte aligned (ldg % 8 == 0), act == NONE, no residual, no folded
-                              LayerNorm; TAIR_ERR_INVALID otherwise.                       */
+                              LayerNorm; TAIR_ERR_INVALID otherwise.  Not on the split-K path of
+                              tair_conv3x3_bf16 either (see `workspace`): a conv whose output image is at most 8x8 with
+                              K >= 4096, given a workspace, returns TAIR_ERR_INVALID for bf16 rows (fp32 rows work).  */
   void* workspace;         /* optional scratch (16-byte aligned, private to the stream) or NULL.  When given and large
                               enough (3 * M * N * 4 bytes), tair_conv3x3_bf16 computes layers whose OUTPUT image is at
                               most 8x8 with K >= 4096 as a 3-way split-K: fp32 partial tiles in the workspace, then

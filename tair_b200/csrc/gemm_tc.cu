@@ -1315,6 +1315,10 @@ int tuned_dispatch(const CUtensorMap& tmA, const void* A, size_t in_bytes, const
   p.tiles_m = (p.M + BM - 1) / BM;
   if (const char* f = getenv("TAIR_GEMM_BN")) {  // bring-up probe only
     const int bn = atoi(f);
+    // a GEGLU weight is interleaved for one tile width (interleave_geglu): any other BN would pair value rows with value rows
+    const int geglu_bn = act == TAIR_ACT_GEGLU ? pick_bn(p.M, p.N, p.num_kb, act) : bn;
+    TAIR_REQUIRE(bn == geglu_bn, "gemm: TAIR_GEMM_BN=%d does not match the GEGLU weight interleave (BN=%d for N=%d)", bn,
+                 geglu_bn, p.N);
     if (const char* sp = getenv("TAIR_GEMM_SPLITS")) {   // probe: needs a caller workspace
       const int splits = atoi(sp);
       if (legal_splitk(p, act, bn, splits) && p.epi.workspace != nullptr &&
