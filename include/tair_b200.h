@@ -13,6 +13,8 @@
  *       `_C.ms_deform_attn_forward`                      -> tair_msda_forward
  *   - terediff/sampler/spaced_sampler.py:141-147,123-131,167-189 (p_sample math)
  *                                                        -> tair_sampler_update
+ *   - DDIM / DPM-Solver++(2M) update (DiffBIR's samplers; not in TAIR)
+ *                                                        -> tair_sampler_multistep_update
  *   - val_patches.py:114-206 (merge_patches_with_overlap) -> tair_blend_tiles
  *   - terediff/model/unet.py:203-223 / util.py:182-193 (GroupNorm32+SiLU)
  *                                                        -> tair_groupnorm_nhwc
@@ -149,6 +151,18 @@ int tair_sampler_update(const float* x, const float* v_cond, const float* v_unco
                         const float* sqrt_alphas_cumprod, const float* sqrt_one_minus_alphas_cumprod,
                         const float* posterior_mean_coef1, const float* posterior_mean_coef2,
                         const float* posterior_variance, int32_t B, int32_t per_sample, void* stream);
+
+/* One multistep (DDIM / DPM-Solver++(2M)) update, all tensors fp32 [B, per_sample]:
+ *   v      = v_uncond ? v_uncond + cfg_scale*(v_cond - v_uncond) : v_cond      (cfg_scale_dev as in tair_sampler_update)
+ *   x0     = P[t]*x - Q[t]*v            (same order of operations as tair_sampler_update)
+ *   x_next = ((b[t]*x0 + a[t]*x) + c[t]*x0_hist) + d[t]*noise
+ *   x0_hist <- x0                        (in place; x0_hist may be NULL only where every c[t] used is 0)
+ * x0_hist is not read for a sample whose c[t] == 0, so stale or NaN history never reaches the result.  x_next must not
+ * alias x, v_cond, v_uncond or x0_hist.  t is the int64 [B] index into the per-step tables (device pointers). */
+int tair_sampler_multistep_update(const float* x, const float* v_cond, const float* v_uncond, float cfg_scale,
+                                  const float* cfg_scale_dev, const float* noise, float* x_next, float* x0_hist,
+                                  const int64_t* t, const float* P, const float* Q, const float* a, const float* b,
+                                  const float* c, const float* d, int32_t B, int32_t per_sample, void* stream);
 
 /* out[b, :] = cos(t*f) || sin(t*f), f_k = exp(-ln(max_period) k/half); t int64 [B]; out bf16 [B, dim]. */
 int tair_timestep_embedding(const int64_t* t, void* out, int32_t B, int32_t dim, float max_period, void* stream);

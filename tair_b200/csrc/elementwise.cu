@@ -2,6 +2,7 @@
 //
 //   tair_sampler_update   : v -> x0 -> posterior mean/variance -> x_{t-1}, optional CFG combine
 //                           (terediff/sampler/spaced_sampler.py:141-147,123-131,149-164,167-189)
+//   tair_sampler_multistep_update: v -> x0 -> DDIM / DPM-Solver++(2M) step with an in-place x0 history
 //   tair_timestep_embedding: cos||sin sinusoidal embedding (terediff/model/util.py:128-148)
 //   tair_nchw_to_nhwc_bf16 / tair_nhwc_to_nchw_f32 : reference (B,C,H,W) fp32 <-> internal [B*H*W, C] bf16
 //   tair_concat_add       : out = [a | b (+ c)] along channels  (decoder skip: controlnet.py:46-50)
@@ -55,6 +56,50 @@ __global__ void sampler_update_kernel(const float* __restrict__ x, const float* 
   out.w = __fadd_rn(__fadd_rn(__fmul_rn(c1, x0.w), __fmul_rn(c2, xv.w)), __fmul_rn(sigma, nz.w));
   *reinterpret_cast<float4*>(x_prev + i4) = out;
   if (x0_out != nullptr) *reinterpret_cast<float4*>(x0_out + i4) = x0;
+}
+
+// DDIM / DPM-Solver++(2M) step: x_next = ((b*x0 + a*x) + c*x0_hist) + d*noise, x0_hist <- x0.  The CFG combine and the
+// x0 line are those of sampler_update_kernel, in the same order.  Each thread reads and then overwrites its own float4 of
+// x0_hist, so the in-place history update has no race.
+__global__ void sampler_multistep_kernel(const float* __restrict__ x, const float* __restrict__ v_cond,
+                                         const float* __restrict__ v_uncond, const float* __restrict__ noise,
+                                         float* __restrict__ x_next, float* __restrict__ x0_hist,
+                                         const int64_t* __restrict__ t, const float* __restrict__ P,
+                                         const float* __restrict__ Q, const float* __restrict__ A,
+                                         const float* __restrict__ Bc, const float* __restrict__ Cc,
+                                         const float* __restrict__ D, float cfg_scale,
+                                         const float* __restrict__ cfg_scale_dev, int per_sample, int total) {
+  pdl_grid_sync();
+  const int i4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+  if (i4 >= total) return;
+  const int b = i4 / per_sample;
+  const int64_t ti = t[b];
+  const float p = P[ti], q = Q[ti], ca = A[ti], cb = Bc[ti], cc = Cc[ti], cd = D[ti];
+  const float4 xv = *reinterpret_cast<const float4*>(x + i4);
+  float4 vv = *reinterpret_cast<const float4*>(v_cond + i4);
+  if (v_uncond != nullptr) {
+    if (cfg_scale_dev != nullptr) cfg_scale = *cfg_scale_dev;
+    const float4 vu = *reinterpret_cast<const float4*>(v_uncond + i4);
+    vv.x = __fadd_rn(vu.x, __fmul_rn(cfg_scale, __fsub_rn(vv.x, vu.x)));
+    vv.y = __fadd_rn(vu.y, __fmul_rn(cfg_scale, __fsub_rn(vv.y, vu.y)));
+    vv.z = __fadd_rn(vu.z, __fmul_rn(cfg_scale, __fsub_rn(vv.z, vu.z)));
+    vv.w = __fadd_rn(vu.w, __fmul_rn(cfg_scale, __fsub_rn(vv.w, vu.w)));
+  }
+  const float4 nz = *reinterpret_cast<const float4*>(noise + i4);
+  // c == 0 is uniform per sample: the history is not read, so a first step never sees stale (or NaN) history
+  float4 h = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (cc != 0.f && x0_hist != nullptr) h = *reinterpret_cast<const float4*>(x0_hist + i4);
+  float4 x0, out;
+  x0.x = __fsub_rn(__fmul_rn(p, xv.x), __fmul_rn(q, vv.x));
+  x0.y = __fsub_rn(__fmul_rn(p, xv.y), __fmul_rn(q, vv.y));
+  x0.z = __fsub_rn(__fmul_rn(p, xv.z), __fmul_rn(q, vv.z));
+  x0.w = __fsub_rn(__fmul_rn(p, xv.w), __fmul_rn(q, vv.w));
+  out.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(cb, x0.x), __fmul_rn(ca, xv.x)), __fmul_rn(cc, h.x)), __fmul_rn(cd, nz.x));
+  out.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(cb, x0.y), __fmul_rn(ca, xv.y)), __fmul_rn(cc, h.y)), __fmul_rn(cd, nz.y));
+  out.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(cb, x0.z), __fmul_rn(ca, xv.z)), __fmul_rn(cc, h.z)), __fmul_rn(cd, nz.z));
+  out.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(cb, x0.w), __fmul_rn(ca, xv.w)), __fmul_rn(cc, h.w)), __fmul_rn(cd, nz.w));
+  *reinterpret_cast<float4*>(x_next + i4) = out;
+  if (x0_hist != nullptr) *reinterpret_cast<float4*>(x0_hist + i4) = x0;
 }
 
 __global__ void timestep_embedding_kernel(const int64_t* __restrict__ t, __nv_bfloat16* __restrict__ out, int B,
@@ -259,6 +304,27 @@ extern "C" int tair_sampler_update(const float* x, const float* v_cond, const fl
       posterior_mean_coef1, posterior_mean_coef2, posterior_variance, cfg_scale, cfg_scale_dev, per_sample, total);
   g_launch_count.fetch_add(1, std::memory_order_relaxed);
   return check_launch("sampler_update_kernel");
+}
+
+extern "C" int tair_sampler_multistep_update(const float* x, const float* v_cond, const float* v_uncond,
+                                             float cfg_scale, const float* cfg_scale_dev, const float* noise,
+                                             float* x_next, float* x0_hist, const int64_t* t, const float* P,
+                                             const float* Q, const float* a, const float* b, const float* c,
+                                             const float* d, int32_t B, int32_t per_sample, void* stream) {
+  TAIR_REQUIRE(x && v_cond && noise && x_next && t, "sampler_multistep_update: NULL pointer");
+  TAIR_REQUIRE(P && Q && a && b && c && d, "sampler_multistep_update: NULL schedule table");
+  TAIR_REQUIRE(B > 0 && per_sample > 0 && per_sample % 4 == 0,
+               "sampler_multistep_update: per_sample must be a multiple of 4");
+  TAIR_REQUIRE(al16(x) && al16(v_cond) && al16(noise) && al16(x_next) && (!v_uncond || al16(v_uncond)) &&
+                   (!x0_hist || al16(x0_hist)), "sampler_multistep_update: tensors must be 16-byte aligned");
+  TAIR_REQUIRE(x_next != x && x_next != v_cond && x_next != v_uncond && x_next != x0_hist,
+               "sampler_multistep_update: x_next must not alias an input");
+  const int total = B * per_sample;
+  const int threads = 256, grid = (total / 4 + threads - 1) / threads;
+  TAIR_LAUNCH((sampler_multistep_kernel), grid, threads, 0, static_cast<cudaStream_t>(stream),
+      x, v_cond, v_uncond, noise, x_next, x0_hist, t, P, Q, a, b, c, d, cfg_scale, cfg_scale_dev, per_sample, total);
+  g_launch_count.fetch_add(1, std::memory_order_relaxed);
+  return check_launch("sampler_multistep_kernel");
 }
 
 extern "C" int tair_timestep_embedding(const int64_t* t, void* out, int32_t B, int32_t dim, float max_period,

@@ -338,6 +338,41 @@ def sampler_update(x, v_cond, noise, t, tables, *, v_uncond=None, cfg_scale: flo
     return out
 
 
+def sampler_multistep_update(x, v_cond, noise, t, tables, *, x0_hist=None, v_uncond=None, cfg_scale: float = 1.0,
+                             cfg_scale_dev=None, out=None):
+    """tables = (P, Q, a, b, c, d): x0 = P[t] x - Q[t] v, x_next = ((b[t] x0 + a[t] x) + c[t] x0_hist) + d[t] noise,
+    then x0_hist <- x0 in place (DDIM / DPM-Solver++(2M)).  fp32 CUDA vectors; t int64 [B].  ``x0_hist`` is not read
+    where c[t] == 0 and may be None only when every c[t] used is 0."""
+    def chk(tt, n):
+        _cuda(tt, n, torch.float32)
+        if not tt.is_contiguous() or tt.shape != x.shape or tt.device != x.device:
+            raise TairError(f"sampler_multistep_update: {n} must be a contiguous fp32 tensor of x's shape on x's device")
+        return tt
+    _cuda(x, "x", torch.float32)
+    for tt, n in ((x, "x"), (v_cond, "v"), (noise, "noise")):
+        chk(tt, n)
+    for tt, n in ((v_uncond, "v_uncond"), (out, "out"), (x0_hist, "x0_hist")):
+        if tt is not None:
+            chk(tt, n)
+    _cuda(t, "t", torch.int64)
+    if cfg_scale_dev is not None:
+        _cuda(cfg_scale_dev, "cfg_scale_dev", torch.float32)
+    B = x.shape[0]
+    if t.numel() != B or not t.is_contiguous():
+        raise TairError("sampler_multistep_update: t must be a contiguous int64 vector with one entry per sample")
+    if len(tables) != 6:
+        raise TairError("sampler_multistep_update: tables must be (P, Q, a, b, c, d)")
+    per = x.numel() // B
+    if out is None:
+        out = torch.empty_like(x)
+    tabs = [_cuda(tb, "schedule table", torch.float32).data_ptr() for tb in tables]
+    rc = _lib.lib().tair_sampler_multistep_update(x.data_ptr(), v_cond.data_ptr(), _ptr(v_uncond), float(cfg_scale),
+                                                  _ptr(cfg_scale_dev), noise.data_ptr(), out.data_ptr(), _ptr(x0_hist),
+                                                  t.data_ptr(), *tabs, B, per, _stream())
+    _lib.check(rc, "tair_sampler_multistep_update")
+    return out
+
+
 def timestep_embedding(t: torch.Tensor, dim: int, max_period: float = 10000.0) -> torch.Tensor:
     _cuda(t, "t", torch.int64)
     out = torch.empty((t.shape[0], dim), device=t.device, dtype=BF16)

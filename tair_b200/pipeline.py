@@ -52,7 +52,11 @@ def restore_image(lq: np.ndarray, cldm, sampler, *, cond_fn: Optional[Callable] 
                   decode_fn: Optional[Callable] = None, cleaner: Optional[Callable] = None, ts_model=None,
                   steps: int = 50, tile_batch: int = 16, cfg_scale: float = 1.0, uncond_fn: Optional[Callable] = None,
                   seed: int = 25, group=None, use_cuda_graph: bool = True, cfg=None) -> torch.Tensor:
-    """lq: (H,W,3) uint8 low-quality image -> (1,3,4H,4W) restored image on every rank."""
+    """lq: (H,W,3) uint8 low-quality image -> (1,3,4H,4W) restored image on every rank.
+
+    ``sampler`` is any sampler of ``tair_b200.sampler``: ``SpacedSampler`` (the reference's 50-step DDPM), or
+    ``DDIMSampler`` / ``DPMSolverSampler`` (one network evaluation per step, usually run with fewer ``steps``).  The
+    step noise is drawn per tile either way, so the result does not depend on ``tile_batch``."""
     import torch.distributed as dist
     dev = next(cldm.parameters()).device
     if cond_fn is None:
