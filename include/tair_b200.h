@@ -15,6 +15,8 @@
  *                                                        -> tair_sampler_update
  *   - DDIM / DPM-Solver++(2M) update (DiffBIR's samplers; not in TAIR)
  *                                                        -> tair_sampler_multistep_update
+ *   - UniPC predictor-corrector update (Zhao et al. 2023; not in TAIR)
+ *                                                        -> tair_sampler_unipc_update
  *   - val_patches.py:114-206 (merge_patches_with_overlap) -> tair_blend_tiles
  *   - terediff/model/unet.py:203-223 / util.py:182-193 (GroupNorm32+SiLU)
  *                                                        -> tair_groupnorm_nhwc
@@ -163,6 +165,25 @@ int tair_sampler_multistep_update(const float* x, const float* v_cond, const flo
                                   const float* cfg_scale_dev, const float* noise, float* x_next, float* x0_hist,
                                   const int64_t* t, const float* P, const float* Q, const float* a, const float* b,
                                   const float* c, const float* d, int32_t B, int32_t per_sample, void* stream);
+
+/* One UniPC step (bh2 data prediction: the UniC corrector of the current point, then the UniP predictor of the next),
+ * all tensors fp32 [B, per_sample]; table is fp32 [N, 16], row t[b] for sample b, columns
+ *   0 P, 1 Q, 2 u, 3 e, 4 f, 5..7 g0..g2, 8 a, 9 b, 10..12 c0..c2, 13..15 unused.
+ *   v      = v_uncond ? v_uncond + cfg_scale*(v_cond - v_uncond) : v_cond      (cfg_scale_dev as in tair_sampler_update)
+ *   x0     = P*x - Q*v                   (same order of operations as tair_sampler_update)
+ *   xc     = 0 (+ u*x) (+ e*x_corr) (+ f*x0) (+ g0*h0) (+ g1*h1) (+ g2*h2)
+ *   x_next = 0 (+ a*xc) (+ b*x0) (+ c0*h0) (+ c1*h1) (+ c2*h2)
+ *   x_corr <- xc;  h_{K-1} <- h_{K-2}, ..., h1 <- h0, h0 <- x0       (in place)
+ * h_k is slot k of x0_hist, a contiguous fp32 [K, B, per_sample] buffer, K in {1, 2, 3}; x is the latent the network
+ * saw (the previous predictor output) and x_corr the corrected latent of the previous step.  The sums are evaluated left
+ * to right, every product and sum rounded to fp32 on its own (no fused multiply-add); a bracketed term is added only
+ * where its coefficient is non-zero (and k < K), so a state value with a zero coefficient is never multiplied (a history
+ * slot may be read only to be shifted on) and stale or NaN state never reaches the result.  A step without correction has u = 1 and e = f = g = 0, so xc = x.  x_next must not
+ * alias an input or state buffer, and x_corr and x0_hist must not alias each other or an input. */
+int tair_sampler_unipc_update(const float* x, const float* v_cond, const float* v_uncond, float cfg_scale,
+                              const float* cfg_scale_dev, float* x_next, float* x_corr, float* x0_hist,
+                              const int64_t* t, const float* table, int32_t K, int32_t B, int32_t per_sample,
+                              void* stream);
 
 /* out[b, :] = cos(t*f) || sin(t*f), f_k = exp(-ln(max_period) k/half); t int64 [B]; out bf16 [B, dim]. */
 int tair_timestep_embedding(const int64_t* t, void* out, int32_t B, int32_t dim, float max_period, void* stream);

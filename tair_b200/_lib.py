@@ -62,6 +62,7 @@ SIGNATURES = {
     "tair_layernorm": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _f32, _vp]),
     "tair_sampler_update": (C.c_int, [_vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp]),
     "tair_sampler_multistep_update": (C.c_int, [_vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp]),
+    "tair_sampler_unipc_update": (C.c_int, [_vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp]),
     "tair_timestep_embedding": (C.c_int, [_vp, _vp, _i32, _i32, _f32, _vp]),
     "tair_nchw_to_nhwc_bf16": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp]),
     "tair_nhwc_to_nchw_f32": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32, _vp]),

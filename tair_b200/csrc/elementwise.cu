@@ -3,6 +3,7 @@
 //   tair_sampler_update   : v -> x0 -> posterior mean/variance -> x_{t-1}, optional CFG combine
 //                           (terediff/sampler/spaced_sampler.py:141-147,123-131,149-164,167-189)
 //   tair_sampler_multistep_update: v -> x0 -> DDIM / DPM-Solver++(2M) step with an in-place x0 history
+//   tair_sampler_unipc_update: v -> x0 -> UniPC corrector + predictor with in-place corrected-latent and x0 histories
 //   tair_timestep_embedding: cos||sin sinusoidal embedding (terediff/model/util.py:128-148)
 //   tair_nchw_to_nhwc_bf16 / tair_nhwc_to_nchw_f32 : reference (B,C,H,W) fp32 <-> internal [B*H*W, C] bf16
 //   tair_concat_add       : out = [a | b (+ c)] along channels  (decoder skip: controlnet.py:46-50)
@@ -100,6 +101,82 @@ __global__ void sampler_multistep_kernel(const float* __restrict__ x, const floa
   out.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(cb, x0.w), __fmul_rn(ca, xv.w)), __fmul_rn(cc, h.w)), __fmul_rn(cd, nz.w));
   *reinterpret_cast<float4*>(x_next + i4) = out;
   if (x0_hist != nullptr) *reinterpret_cast<float4*>(x0_hist + i4) = x0;
+}
+
+// acc + c*v per component, unfused (__fmul_rn then __fadd_rn)
+__device__ __forceinline__ float4 add_scaled(float4 acc, float c, float4 v) {
+  return make_float4(__fadd_rn(acc.x, __fmul_rn(c, v.x)), __fadd_rn(acc.y, __fmul_rn(c, v.y)),
+                     __fadd_rn(acc.z, __fmul_rn(c, v.z)), __fadd_rn(acc.w, __fmul_rn(c, v.w)));
+}
+
+// UniPC step (UniC corrector, then UniP predictor) from one packed [N, 16] table row
+//   P Q | u e f g0 g1 g2 | a b c0 c1 c2 | pad:
+//   x0     = P*x - Q*v                                                (the x0 line of sampler_update_kernel)
+//   xc     = 0 (+ u*x) (+ e*xc_prev) (+ f*x0) (+ g0*h0) (+ g1*h1) (+ g2*h2)
+//   x_next = 0 (+ a*xc) (+ b*x0) (+ c0*h0) (+ c1*h1) (+ c2*h2)
+// evaluated left to right in fp32, each product and sum rounded on its own, and each bracketed term added only where its
+// coefficient is non-zero (k < K for the history terms).  The coefficients are uniform per sample, so the branches are
+// too, and a state value whose coefficient is 0 is never multiplied (a history slot may be read only to be shifted
+// on): stale or NaN state never reaches the result.  Then, in
+// place: xc_prev <- xc and h_{K-1} <- h_{K-2}, ..., h1 <- h0, h0 <- x0 (h_k is slot k of x0_hist, `total` floats apart).
+// Each thread reads and then overwrites only its own float4 of every state buffer, so the update has no race.
+__global__ void sampler_unipc_kernel(const float* __restrict__ x, const float* __restrict__ v_cond,
+                                     const float* __restrict__ v_uncond, float* __restrict__ x_next,
+                                     float* __restrict__ x_corr, float* __restrict__ x0_hist,
+                                     const int64_t* __restrict__ t, const float* __restrict__ table, int K,
+                                     float cfg_scale, const float* __restrict__ cfg_scale_dev, int per_sample,
+                                     int total) {
+  pdl_grid_sync();
+  const int i4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+  if (i4 >= total) return;
+  const int b = i4 / per_sample;
+  const float4* row = reinterpret_cast<const float4*>(table + t[b] * 16);
+  const float4 r0 = row[0], r1 = row[1], r2 = row[2], r3 = row[3];
+  const float p = r0.x, q = r0.y, cu = r0.z, ce = r0.w, cf = r1.x, ca = r2.x, cb = r2.y;
+  const float g[3] = {r1.y, r1.z, r1.w}, c[3] = {r2.z, r2.w, r3.x};
+  const float4 xv = *reinterpret_cast<const float4*>(x + i4);
+  float4 vv = *reinterpret_cast<const float4*>(v_cond + i4);
+  if (v_uncond != nullptr) {
+    if (cfg_scale_dev != nullptr) cfg_scale = *cfg_scale_dev;
+    const float4 vu = *reinterpret_cast<const float4*>(v_uncond + i4);
+    vv.x = __fadd_rn(vu.x, __fmul_rn(cfg_scale, __fsub_rn(vv.x, vu.x)));
+    vv.y = __fadd_rn(vu.y, __fmul_rn(cfg_scale, __fsub_rn(vv.y, vu.y)));
+    vv.z = __fadd_rn(vu.z, __fmul_rn(cfg_scale, __fsub_rn(vv.z, vu.z)));
+    vv.w = __fadd_rn(vu.w, __fmul_rn(cfg_scale, __fsub_rn(vv.w, vu.w)));
+  }
+  float4 x0;
+  x0.x = __fsub_rn(__fmul_rn(p, xv.x), __fmul_rn(q, vv.x));
+  x0.y = __fsub_rn(__fmul_rn(p, xv.y), __fmul_rn(q, vv.y));
+  x0.z = __fsub_rn(__fmul_rn(p, xv.z), __fmul_rn(q, vv.z));
+  x0.w = __fsub_rn(__fmul_rn(p, xv.w), __fmul_rn(q, vv.w));
+  // a history slot is loaded where a coefficient uses it, or where the shift moves it on (it is then never multiplied)
+  float4 h[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    h[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (k < K && (k + 1 < K || g[k] != 0.f || c[k] != 0.f))
+      h[k] = *reinterpret_cast<const float4*>(x0_hist + (size_t)k * total + i4);
+  }
+  const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+  float4 xc = zero;
+  if (cu != 0.f) xc = add_scaled(xc, cu, xv);
+  if (ce != 0.f) xc = add_scaled(xc, ce, *reinterpret_cast<const float4*>(x_corr + i4));
+  if (cf != 0.f) xc = add_scaled(xc, cf, x0);
+#pragma unroll
+  for (int k = 0; k < 3; ++k)
+    if (k < K && g[k] != 0.f) xc = add_scaled(xc, g[k], h[k]);
+  float4 out = zero;
+  if (ca != 0.f) out = add_scaled(out, ca, xc);
+  if (cb != 0.f) out = add_scaled(out, cb, x0);
+#pragma unroll
+  for (int k = 0; k < 3; ++k)
+    if (k < K && c[k] != 0.f) out = add_scaled(out, c[k], h[k]);
+  *reinterpret_cast<float4*>(x_next + i4) = out;
+  *reinterpret_cast<float4*>(x_corr + i4) = xc;
+#pragma unroll
+  for (int k = 2; k >= 1; --k)
+    if (k < K) *reinterpret_cast<float4*>(x0_hist + (size_t)k * total + i4) = h[k - 1];
+  *reinterpret_cast<float4*>(x0_hist + i4) = x0;
 }
 
 __global__ void timestep_embedding_kernel(const int64_t* __restrict__ t, __nv_bfloat16* __restrict__ out, int B,
@@ -325,6 +402,37 @@ extern "C" int tair_sampler_multistep_update(const float* x, const float* v_cond
       x, v_cond, v_uncond, noise, x_next, x0_hist, t, P, Q, a, b, c, d, cfg_scale, cfg_scale_dev, per_sample, total);
   g_launch_count.fetch_add(1, std::memory_order_relaxed);
   return check_launch("sampler_multistep_kernel");
+}
+
+// [a, a + na) and [b, b + nb) share a float (nb == 0 or b == NULL: no overlap)
+static inline bool overlaps(const float* a, size_t na, const float* b, size_t nb) {
+  return a != nullptr && b != nullptr && na && nb && a < b + nb && b < a + na;
+}
+
+extern "C" int tair_sampler_unipc_update(const float* x, const float* v_cond, const float* v_uncond, float cfg_scale,
+                                         const float* cfg_scale_dev, float* x_next, float* x_corr, float* x0_hist,
+                                         const int64_t* t, const float* table, int32_t K, int32_t B,
+                                         int32_t per_sample, void* stream) {
+  TAIR_REQUIRE(x && v_cond && x_next && x_corr && x0_hist && t && table, "sampler_unipc_update: NULL pointer");
+  TAIR_REQUIRE(K >= 1 && K <= 3, "sampler_unipc_update: history depth K must be 1, 2 or 3 (got %d)", (int)K);
+  TAIR_REQUIRE(B > 0 && per_sample > 0 && per_sample % 4 == 0,
+               "sampler_unipc_update: per_sample must be a multiple of 4");
+  TAIR_REQUIRE(al16(x) && al16(v_cond) && al16(x_next) && al16(x_corr) && al16(x0_hist) && al16(table) &&
+                   (!v_uncond || al16(v_uncond)), "sampler_unipc_update: tensors must be 16-byte aligned");
+  const size_t n = (size_t)B * per_sample, nh = (size_t)K * n;
+  TAIR_REQUIRE(!overlaps(x_next, n, x, n) && !overlaps(x_next, n, v_cond, n) && !overlaps(x_next, n, v_uncond, n) &&
+                   !overlaps(x_next, n, x_corr, n) && !overlaps(x_next, n, x0_hist, nh),
+               "sampler_unipc_update: x_next must not alias an input or state buffer");
+  TAIR_REQUIRE(!overlaps(x_corr, n, x0_hist, nh) && !overlaps(x_corr, n, x, n) && !overlaps(x_corr, n, v_cond, n) &&
+                   !overlaps(x_corr, n, v_uncond, n) && !overlaps(x0_hist, nh, x, n) &&
+                   !overlaps(x0_hist, nh, v_cond, n) && !overlaps(x0_hist, nh, v_uncond, n),
+               "sampler_unipc_update: x_corr and x0_hist must not alias each other or an input");
+  const int total = B * per_sample;
+  const int threads = 256, grid = (total / 4 + threads - 1) / threads;
+  TAIR_LAUNCH((sampler_unipc_kernel), grid, threads, 0, static_cast<cudaStream_t>(stream),
+      x, v_cond, v_uncond, x_next, x_corr, x0_hist, t, table, (int)K, cfg_scale, cfg_scale_dev, per_sample, total);
+  g_launch_count.fetch_add(1, std::memory_order_relaxed);
+  return check_launch("sampler_unipc_kernel");
 }
 
 extern "C" int tair_timestep_embedding(const int64_t* t, void* out, int32_t B, int32_t dim, float max_period,

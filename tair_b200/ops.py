@@ -373,6 +373,49 @@ def sampler_multistep_update(x, v_cond, noise, t, tables, *, x0_hist=None, v_unc
     return out
 
 
+def sampler_unipc_update(x, v_cond, t, table, *, x_corr, x0_hist, v_uncond=None, cfg_scale: float = 1.0,
+                         cfg_scale_dev=None, out=None):
+    """One UniPC step from the packed fp32 [N, 16] ``table`` (columns P, Q, u, e, f, g0..g2, a, b, c0..c2, padding):
+    x0 = P[t] x - Q[t] v, xc = u x + e x_corr + f x0 + sum_k g_k h_k, x_next = a xc + b x0 + sum_k c_k h_k, then
+    x_corr <- xc and the history shifts (h0 <- x0, h_k <- h_{k-1}) in place.  ``x0_hist`` is a contiguous fp32
+    [K, *x.shape] buffer, K in {1, 2, 3}; t int64 [B].  A state term enters a sum only where its coefficient is non-zero;
+    the fp32 evaluation order is documented at ``tair_sampler_unipc_update`` in include/tair_b200.h."""
+    def chk(tt, n, shape):
+        _cuda(tt, n, torch.float32)
+        if not tt.is_contiguous() or tt.shape != shape or tt.device != x.device:
+            raise TairError(f"sampler_unipc_update: {n} must be a contiguous fp32 tensor of shape {tuple(shape)} on "
+                            f"x's device")
+        return tt
+    _cuda(x, "x", torch.float32)
+    for tt, n in ((x, "x"), (v_cond, "v"), (x_corr, "x_corr")):
+        chk(tt, n, x.shape)
+    for tt, n in ((v_uncond, "v_uncond"), (out, "out")):
+        if tt is not None:
+            chk(tt, n, x.shape)
+    _cuda(x0_hist, "x0_hist", torch.float32)
+    K = x0_hist.shape[0] if x0_hist.dim() == x.dim() + 1 else 0
+    if not 1 <= K <= 3:
+        raise TairError("sampler_unipc_update: x0_hist must have shape (K, *x.shape) with K in {1, 2, 3}")
+    chk(x0_hist, "x0_hist", (K,) + tuple(x.shape))
+    _cuda(t, "t", torch.int64)
+    if cfg_scale_dev is not None:
+        _cuda(cfg_scale_dev, "cfg_scale_dev", torch.float32)
+    B = x.shape[0]
+    if t.numel() != B or not t.is_contiguous():
+        raise TairError("sampler_unipc_update: t must be a contiguous int64 vector with one entry per sample")
+    _cuda(table, "table", torch.float32)
+    if table.dim() != 2 or table.shape[1] != 16 or not table.is_contiguous() or table.device != x.device:
+        raise TairError("sampler_unipc_update: table must be a contiguous fp32 [N, 16] tensor on x's device")
+    per = x.numel() // B
+    if out is None:
+        out = torch.empty_like(x)
+    rc = _lib.lib().tair_sampler_unipc_update(x.data_ptr(), v_cond.data_ptr(), _ptr(v_uncond), float(cfg_scale),
+                                              _ptr(cfg_scale_dev), out.data_ptr(), x_corr.data_ptr(),
+                                              x0_hist.data_ptr(), t.data_ptr(), table.data_ptr(), K, B, per, _stream())
+    _lib.check(rc, "tair_sampler_unipc_update")
+    return out
+
+
 def timestep_embedding(t: torch.Tensor, dim: int, max_period: float = 10000.0) -> torch.Tensor:
     _cuda(t, "t", torch.int64)
     out = torch.empty((t.shape[0], dim), device=t.device, dtype=BF16)

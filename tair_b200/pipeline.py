@@ -55,7 +55,8 @@ def restore_image(lq: np.ndarray, cldm, sampler, *, cond_fn: Optional[Callable] 
     """lq: (H,W,3) uint8 low-quality image -> (1,3,4H,4W) restored image on every rank.
 
     ``sampler`` is any sampler of ``tair_b200.sampler``: ``SpacedSampler`` (the reference's 50-step DDPM), or
-    ``DDIMSampler`` / ``DPMSolverSampler`` (one network evaluation per step, usually run with fewer ``steps``).  The
+    ``DDIMSampler`` / ``DPMSolverSampler`` / ``UniPCSampler`` (one network evaluation per step, usually run with fewer
+    ``steps``).  The
     step noise is drawn per tile either way, so the result does not depend on ``tile_batch``."""
     import torch.distributed as dist
     dev = next(cldm.parameters()).device

@@ -1,9 +1,10 @@
-"""Spaced-50 vs DDIM-25 vs DPM-Solver++(2M)-20 at the bench batch (B=16, synthetic weights), in one process, alternating.
+"""Spaced-50 vs DDIM-25 vs DPM-Solver++(2M)-20 vs UniPC-2 at 10 and 15 steps at the bench batch (B=16, synthetic weights),
+in one process, alternating.
 
 For each sampler: a whole `sample` run (ControlNet + UNet + update per step, CUDA graph) and a whole `val_sample` run
 (+ TESTR head, detection post-processing, prompt and CLIP re-encode per step), timed with a host clock around work that
-ends in a device synchronise.  Reports ms per step, s per batch and patches/s, and the fused multistep update kernel
-against tair_sampler_update (CUDA events around graph replays of 200 back-to-back launches on the [16, 4, 64, 64] latent,
+ends in a device synchronise.  Reports ms per step, s per batch and patches/s, and the fused multistep and UniPC update
+kernels against tair_sampler_update (CUDA events around graph replays of 200 back-to-back launches on the [16, 4, 64, 64] latent,
 which stays in L2).  The GPU name and power limit are read in the same run.  Prints the result as JSON, and writes it
 to the file given with --out."""
 import argparse
@@ -25,7 +26,7 @@ from tair_b200.init import nondegenerate_init_  # noqa: E402
 from tair_b200.model import ControlLDM  # noqa: E402
 from tair_b200.model.clip import FrozenOpenCLIPEmbedder  # noqa: E402
 from tair_b200.model.gaussian_diffusion import val_diffusion  # noqa: E402
-from tair_b200.sampler import DDIMSampler, DPMSolverSampler, SpacedSampler  # noqa: E402
+from tair_b200.sampler import DDIMSampler, DPMSolverSampler, SpacedSampler, UniPCSampler  # noqa: E402
 from tair_b200.testr import TransformerDetector, default_cfg  # noqa: E402
 
 B, REPS = 16, int(os.environ.get("REPS", "3"))
@@ -62,7 +63,9 @@ def main():
     nondegenerate_init_(det, 99)
     betas = val_diffusion().betas
     configs = [("spaced", SpacedSampler(betas), 50), ("ddim", DDIMSampler(betas), 25),
-               ("dpmpp2m", DPMSolverSampler(betas), 20)]
+               ("dpmpp2m", DPMSolverSampler(betas), 20),
+               # one instance per step count: a schedule change re-allocates the tables and drops the captured graphs
+               ("unipc2_", UniPCSampler(betas, order=2), 10), ("unipc2_", UniPCSampler(betas, order=2), 15)]
     g = torch.Generator(device=dev).manual_seed(0)
     x_T = torch.randn((B, 4, 64, 64), device=dev, generator=g)
     c_img = torch.randn((B, 4, 64, 64), device=dev, generator=g)
@@ -82,19 +85,19 @@ def main():
         assert torch.isfinite(z).all()
         return time.perf_counter() - t0
 
-    times = {(name, kind): [] for name, _, _ in configs for kind in ("sample", "val_sample")}
+    times = {(name + str(n), kind): [] for name, _, n in configs for kind in ("sample", "val_sample")}
     for name, s, n in configs:           # warm-up: graph capture, autotuning, CLIP cache
         for kind in ("sample", "val_sample"):
             run(kind, s, n)
     for _ in range(REPS):
         for name, s, n in configs:
             for kind in ("sample", "val_sample"):
-                times[name, kind].append(run(kind, s, n))
+                times[name + str(n), kind].append(run(kind, s, n))
 
     res = {"batch": B, "reps": REPS, "gpu_before": info_before, "runs": {}}
     for name, s, n in configs:
         for kind in ("sample", "val_sample"):
-            ts = times[name, kind]
+            ts = times[name + str(n), kind]
             best, med = min(ts), sorted(ts)[len(ts) // 2]
             res["runs"][f"{name}{n}_{kind}"] = {
                 "steps": n, "s_per_batch_all": [round(t, 4) for t in ts], "s_per_batch_median": round(med, 4),
@@ -112,6 +115,11 @@ def main():
     ms.to(dev)
     out = torch.empty_like(x)
     hist = ms.x0_history(x)
+    uni = {}
+    for order in (2, 3):    # a corrected step of full order: every state slot is read
+        u = uni[order] = UniPCSampler(betas, order=order)
+        u.make_schedule(20)
+        u.to(dev)
 
     def ev(fn, n=200, reps=10):
         """us per launch: n launches captured in one CUDA graph, replayed reps times (no host overhead per launch)."""
@@ -135,6 +143,10 @@ def main():
         kern.setdefault("sampler_update_us", []).append(ev(lambda: ops.sampler_update(x, v, nz, t, spaced._tables(), out=out)))
         kern.setdefault("sampler_multistep_update_us", []).append(
             ev(lambda: ops.sampler_multistep_update(x, v, nz, t, ms._tables(), x0_hist=hist, out=out)))
+        for order, u in uni.items():
+            xc, h = u.state_buffers(x)
+            kern.setdefault(f"sampler_unipc_update_k{order}_us", []).append(
+                ev(lambda: ops.sampler_unipc_update(x, v, t, u.unipc_table, x_corr=xc, x0_hist=h, out=out)))
     res["update_kernel"] = {k: [round(u, 3) for u in vals] for k, vals in kern.items()}
     res["update_kernel"]["note"] = ("per launch, 200 launches per CUDA graph replayed 10 times; "
                                     "[16,4,64,64] fp32 operands stay in L2")
